@@ -5,6 +5,7 @@
     python bench.py --workload {vga_lightglue,mp1_lightglue,seq_superglue,superpoint_only,small_stop}
     python bench.py --impl reference --gpus N --steps K ...        # the reference algorithm on the host CPU cores
     python bench.py --scaling strong --frames F                    # ONE fixed job through the L2 seam, pairs sharded p mod world
+    python bench.py --steps K --warmup W --dump-outputs DIR        # also write what the last timed step computed (dump_outputs)
 
 Workloads (config.workload):
   vga_lightglue   (default; the driver's line) steady state of BASELINE.json configs[3] with the deep_front_end.yaml matcher: synthetic
@@ -16,7 +17,7 @@ Workloads (config.workload):
   small_stop      launch-bound regime: 1024 keypoints, 'stop' weights (early exit at layer 4-5, pruning on).  STEP = 40 pairs.
 Pairs shard across GPUs with no data-path collective (one weight broadcast at start-up); per-GPU work is fixed => "weak" scaling.
 `--scaling strong` instead times one fixed job (F frames, lookahead 20) through B200CorrespondenceGenerator (two-view verification run under the matching),
-including image (re-)detection on every rank and the final gather, wall-clock on rank 0.
+including image (re-)detection on every rank and the final gather, wall-clock on rank 0; each of the --steps steps is one whole job.
 
 `value` times the device-resident path (frames already in HBM, features / matches stay in HBM, only per-pair scalars come back);
 `e2e` times the same step through the GTSfM plugin classes with HOST numpy buffers, so every H2D / D2H copy the per-call API
@@ -257,7 +258,7 @@ def run_reference(args):
         return
     w = WORKLOADS[args.workload]
     vals, cb = [], None
-    for i in range(max(1, min(args.steps, 2))):  # each "step" is one bounded sweep of the layouts (tens of seconds)
+    for i in range(args.steps):  # each "step" is one bounded sweep of the layouts (tens of seconds)
         cb = cpu_baseline(args.workload, quick=False)
         vals.append(cb["value"])
     value = float(np.mean(vals))
@@ -305,6 +306,49 @@ def _broadcast_weights(sds, world, dev):
             off += n
 
 
+DUMP_BYTES = 64 * 10**6  # --dump-outputs writes at most this much
+
+
+def dump_outputs(out: Path, step: dict) -> None:
+    """Write what the last timed step returned to its caller, as .npy files under `out` (float32, or float64 where a float32
+    could not hold every value exactly):
+      keypoints (N, 2), scores (N,), keypoints_per_frame (F,)   the step's new frames, concatenated in frame order
+      descriptors (D, 256), descriptor_rows (D,)                 the rows of the concatenated descriptors: all N, or a fixed seeded
+                                                                 sample of them where all would not fit in DUMP_BYTES
+      matches (M, 2), matches_per_pair (P,), stop_layer (P,)     pairs ordered by (new frame, window slot); stop_layer for LightGlue
+      inlier_mask (M,), num_inliers (P,), essential (P, 3, 3), rotation (P, 3, 3), translation (P, 3)
+                                                                 each pair's verification; NaN where it found no model"""
+    import torch
+
+    feats = step["features"]
+    arrays = {"keypoints": torch.cat([f.kp for f in feats]).float().cpu().numpy(),
+              "scores": torch.cat([f.score for f in feats]).float().cpu().numpy(),
+              "keypoints_per_frame": np.array([len(f) for f in feats], np.float64)}
+    pairs = [step["pairs"][k] for k in sorted(step.get("pairs", {}))]
+    if pairs:
+        arrays["matches"] = np.concatenate([p["matches"].cpu().numpy().reshape(-1, 2) for p in pairs]).astype(np.float64)
+        arrays["matches_per_pair"] = np.array([p["matches"].shape[0] for p in pairs], np.float64)
+        if "stop" in pairs[0]:
+            arrays["stop_layer"] = np.array([p["stop"] for p in pairs], np.float64)
+        nan = lambda shape: np.full(shape, np.nan)  # noqa: E731
+        verified = [p["verify"] for p in pairs]
+        arrays["inlier_mask"] = np.concatenate([v[4].cpu().numpy() for v in verified]).astype(np.float32)
+        arrays["num_inliers"] = np.array([v[3] for v in verified], np.float64)
+        arrays["essential"] = np.stack([nan((3, 3)) if v[0] is None else v[0] for v in verified]).astype(np.float64)
+        arrays["rotation"] = np.stack([nan((3, 3)) if v[1] is None else v[1] for v in verified]).astype(np.float64)
+        arrays["translation"] = np.stack([nan(3) if v[2] is None else np.asarray(v[2]).ravel() for v in verified]).astype(np.float64)
+    n = int(arrays["keypoints"].shape[0])
+    fit = (DUMP_BYTES - 4096 - sum(a.nbytes for a in arrays.values())) // (256 * 4 + 8)  # 4096: room for the .npy headers
+    rows = np.arange(n) if n <= fit else np.sort(np.random.default_rng(0).choice(n, fit, replace=False))
+    desc = torch.cat([f.desc for f in feats])
+    arrays["descriptors"] = desc[torch.from_numpy(rows).to(desc.device)].float().cpu().numpy()
+    arrays["descriptor_rows"] = rows.astype(np.float64)
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_BYTES
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out / f"{name}.npy", a)
+
+
 def run_cuda(args):
     import torch
     import torch.distributed as dist
@@ -347,43 +391,56 @@ def run_cuda(args):
 
     stats_lock = threading.Lock()
 
-    def step_device(c):
+    def step_device(c, record=None):
+        """One step.  `record` (a dict) receives what the step hands its caller: the new frames' features in order, and per pair
+        (key (new frame, window slot)) the matches, the LightGlue stop layer and the verification result."""
         pending = []
         if not w["matcher"]:  # detect-describe only: every frame of the step enqueued before the first count is read
             for f in fe.detect_many([frames_dev[(c + j) % len(frames_dev)] for j in range(NEW_FRAMES)]):
                 stats["keypoints"] += len(f)
                 stats["frames"] += 1
+                if record is not None:
+                    record.setdefault("features", []).append(f)
             return
         for j in range(NEW_FRAMES):
             f = fe.detect(frames_dev[(c + j) % len(frames_dev)])
             stats["keypoints"] += len(f)
             stats["frames"] += 1
+            if record is not None:
+                record.setdefault("features", []).append(f)
             if not w["matcher"]:
                 continue
             prevs = list(window)
             if w["matcher"] == "lightglue":
                 # lock-step batches of 8 pairs (b2_lightglue_match_batched_dev) over MATCH_LANES concurrent LightGlue instances;
                 # a batch's verifications are queued the moment it completes and overlap the other batches' matcher kernels
-                def on_chunk(c0, res, prevs=prevs, f=f):
+                def on_chunk(c0, res, prevs=prevs, f=f, j=j):
                     with stats_lock:
-                        for prev, (m, stop) in zip(prevs[c0:c0 + len(res)], res):
-                            pending.append(fe.verify_async(prev, f, m, cal, cal, THR_PX))
+                        for i, (prev, (m, stop)) in enumerate(zip(prevs[c0:c0 + len(res)], res)):
+                            pending.append(((j, c0 + i), fe.verify_async(prev, f, m, cal, cal, THR_PX)))
                             stats["matches"] += int(m.shape[0])
                             stats["stops"] += stop
                             stats["pairs"] += 1
+                            if record is not None:
+                                record.setdefault("pairs", {})[(j, c0 + i)] = {"matches": m, "stop": stop}
 
                 fe.match_many([(prev, f) for prev in prevs], on_chunk=on_chunk)
             else:
-                def on_pair(i, m, prevs=prevs, f=f):  # a pair's verification is queued the moment its matches exist
+                def on_pair(i, m, prevs=prevs, f=f, j=j):  # a pair's verification is queued the moment its matches exist
                     with stats_lock:
-                        pending.append(fe.verify_async(prevs[i], f, m, cal, cal, THR_PX))
+                        pending.append(((j, i), fe.verify_async(prevs[i], f, m, cal, cal, THR_PX)))
                         stats["matches"] += int(m.shape[0])
                         stats["pairs"] += 1
+                        if record is not None:
+                            record.setdefault("pairs", {})[(j, i)] = {"matches": m}
 
                 fe.match_superglue_many([(prev, f) for prev in prevs], on_pair=on_pair)
             window.append(f)
-        for fut in pending:  # every verification result is collected inside the step
-            stats["inliers"] += fut.result()[3]
+        for key, fut in pending:  # every verification result is collected inside the step
+            res = fut.result()
+            stats["inliers"] += res[3]
+            if record is not None:
+                record["pairs"][key]["verify"] = res
 
     for _ in range(args.warmup):
         step_device(cursor)
@@ -407,14 +464,14 @@ def run_cuda(args):
     # same number of steps.  Default (graph off): the dominant kernel is timed live inside the timed pass.
     in_graph = os.environ.get("B2_SP_GRAPH") == "1" and w["dominant"].startswith(("k_conv", "k_nms", "k_head"))
 
-    def timed_pass(c):
+    def timed_pass(c, record=None):
         tot = 0.0
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        for _ in range(args.steps):
+        for s in range(args.steps):
             flush.fill_(1)  # L2 flush, outside the timed span
             torch.cuda.synchronize()
             e0.record()
-            step_device(c)
+            step_device(c, record if s == args.steps - 1 else None)
             e1.record()
             torch.cuda.synchronize()
             tot += e0.elapsed_time(e1)
@@ -423,10 +480,13 @@ def run_cuda(args):
 
     if not in_graph:
         fe.profile_start(w["dominant"])
-    total_ms, cursor = timed_pass(cursor)
+    last_step = {} if args.dump_outputs and rank == 0 else None
+    total_ms, cursor = timed_pass(cursor, last_step)
     if not in_graph:
         k_ms, k_launches, k_work = fe.profile_stop()
         prof_total_ms = total_ms
+    if last_step is not None:  # before any later step can reuse the matcher's output buffers
+        dump_outputs(Path(args.dump_outputs), last_step)
     launches = fe.launch_count() - launches0 + (fe._vctx.launch_count() - vlaunch0 if fe._vctx else 0)
     if in_graph:
         keep = dict(stats)
@@ -635,16 +695,19 @@ def run_strong(args):
             dist.barrier()
         torch.cuda.synchronize()
 
-    barrier()
-    t0 = time.perf_counter()
-    kps, matches = gen.generate_correspondences(None, images, graph, verify_with=({i: cal for i in range(F)}, THR_PX))
-    t_corr = time.perf_counter() - t0
-    fe = gen._front_end()
-    feats = gen.last_device_features
-    res = gen.last_two_view  # this rank's shard, verified under the matching (B200TwoViewBatch semantics)
-    n_ok = sum(1 for r in res.values() if r.i2Ri1 is not None)
-    barrier()
-    wall = time.perf_counter() - t0
+    wall = t_corr = 0.0
+    for _ in range(args.steps):  # one step = the whole job
+        barrier()
+        t0 = time.perf_counter()
+        kps, matches = gen.generate_correspondences(None, images, graph, verify_with=({i: cal for i in range(F)}, THR_PX))
+        t_corr += time.perf_counter() - t0
+        fe = gen._front_end()
+        feats = gen.last_device_features
+        res = gen.last_two_view  # this rank's shard, verified under the matching (B200TwoViewBatch semantics)
+        n_ok = sum(1 for r in res.values() if r.i2Ri1 is not None)
+        barrier()
+        wall += time.perf_counter() - t0
+    wall, t_corr = wall / args.steps, t_corr / args.steps  # per job
     tt = torch.tensor([wall, t_corr, float(gen.last_detections), float(n_ok)], dtype=torch.float64, device=dev)
     if world > 1:
         mx = tt.clone()
@@ -659,7 +722,7 @@ def run_strong(args):
         cfg["workload"] = (f"strong scaling: ONE job of {F} synthetic 640x480 frames, Sequential lookahead 20 = {len(graph)} pairs (BASELINE configs[3] shape; "
                            f"F = 500 gives its 9 790-pair graph), B200CorrespondenceGenerator with the two-view verification run under the matching, pairs sharded p mod world")
         line = {
-            "metric": "image_pairs_per_sec", "value": len(graph) / wall, "unit": "pairs/s", "n_gpus": world, "steps": 1, "warmup": 1,
+            "metric": "image_pairs_per_sec", "value": len(graph) / wall, "unit": "pairs/s", "n_gpus": world, "steps": args.steps, "warmup": 1,
             "ms_per_step": wall * 1e3, "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": cfg, "gpu_launches": int(fe.launch_count()),
             "strong": {"pairs": len(graph), "frames": F, "wall_s": wall, "correspondence_s_max_rank": t_corr,
@@ -690,7 +753,13 @@ def main():
                     help="opt-in mode: the reference's CUDA numerics for attention (fp16 flash SDPA, one MMA per product); NOT the "
                          "parity-pinned default - the line says so in config.matcher")
     ap.add_argument("--lg-batch", type=int, default=0, help="experiments: pairs per lock-step LightGlue batch inside the library (0 = default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (see dump_outputs; rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "cuda" or args.scaling != "weak"):
+        ap.error("--dump-outputs applies to the CUDA arm's weak-scaling steps")
     global FP16_ATTN
     FP16_ATTN = bool(args.fp16_attention)
     if args.impl == "reference":

@@ -1,4 +1,4 @@
-"""TEST INFRASTRUCTURE — generates tests/golden/*.npz by running the UNMODIFIED reference in the build container.
+"""TEST INFRASTRUCTURE — generates tests/golden/*.npz and gtsfm_bases.json by running the UNMODIFIED reference in the build container.
 
     python -m oracle.make_golden            # needs /root/reference; not runnable on the GPU box
 
@@ -414,6 +414,61 @@ def golden_netvlad():
     np.savez_compressed(OUT / "netvlad.npz", **out)
 
 
+GTSFM_BASES_SCRIPT = """
+import inspect, json, sys, types
+sys.path.insert(0, sys.argv[1])
+class _Stub(types.ModuleType):  # gtsam / dask / hydra are not installable offline; nothing recorded here comes from them
+    def __getattr__(self, n):
+        if n.startswith("__"): raise AttributeError(n)
+        return type(n, (), {"__init__": lambda self, *a, **k: None})
+for name in ("gtsam", "gtsam.noiseModel", "dask", "dask.distributed", "distributed", "hydra", "hydra.utils", "omegaconf"):
+    sys.modules[name] = _Stub(name)
+sys.modules["gtsam"].noiseModel = sys.modules["gtsam.noiseModel"]
+from gtsfm.common.image import Image
+from gtsfm.common.keypoints import Keypoints
+from gtsfm.frontend.detector_descriptor.detector_descriptor_base import DetectorDescriptorBase
+from gtsfm.frontend.matcher.matcher_base import MatcherBase
+from gtsfm.frontend.verifier.verifier_base import VerifierBase
+from gtsfm.ui.gtsfm_process import GTSFMProcess
+
+def params(f):
+    return [[p.name, None if p.default is p.empty else repr(p.default)] for p in inspect.signature(f).parameters.values()]
+
+def methods(cls):
+    return {n: params(f) for n, f in vars(cls).items() if inspect.isfunction(f) and (not n.startswith("_") or n == "__init__")}
+
+def base_state(cls, *args):  # the attributes the base's own __init__ sets for these constructor arguments
+    stub = type("Probe", (cls,), {n: (lambda *a, **k: None) for n in cls.__abstractmethods__})
+    return {k: repr(v) for k, v in vars(stub(*args)).items()}
+
+bases, plugins = {}, {}
+for cls in (DetectorDescriptorBase, MatcherBase, VerifierBase):
+    bases[cls.__name__] = dict(module=cls.__module__, init=params(cls.__init__) if "__init__" in vars(cls) else None,
+                               abstract={n: params(getattr(cls, n)) for n in sorted(cls.__abstractmethods__)})
+plugins["B200SuperPointDetectorDescriptor"] = dict(base="DetectorDescriptorBase", state=base_state(DetectorDescriptorBase, 5000))
+plugins["B200LightGlueMatcher"] = dict(base="MatcherBase", state=base_state(MatcherBase))
+plugins["B200SuperGlueMatcher"] = dict(base="MatcherBase", state=base_state(MatcherBase))
+probe = type("B200Ransac", (VerifierBase,), {n: (lambda *a, **k: None) for n in VerifierBase.__abstractmethods__})
+plugins["B200Ransac"] = dict(base="VerifierBase", state=base_state(VerifierBase, True, 4), repr=repr(probe(True, 4)))
+out = dict(bases=bases, plugins=plugins,
+           process=dict(module=GTSFMProcess.__module__, name=GTSFMProcess.__name__, abstract=sorted(GTSFMProcess.__abstractmethods__)),
+           keypoints=dict(module=Keypoints.__module__, methods=methods(Keypoints)),
+           image=dict(module=Image.__module__, methods=methods(Image)))
+print(json.dumps(out, indent=1, sort_keys=True))
+"""
+
+
+def golden_gtsfm_bases():
+    """The reference's plugin API (the abstract bases GTSfM's front end instantiates through Hydra, Keypoints, Image): module
+    paths, abstract methods and their parameters, what each base's __init__ stores, and the verifier repr that keys GTSfM's
+    two-view cache.  Read in a subprocess, with empty stand-ins for gtsam / dask / hydra, so they never reach this process."""
+    import subprocess
+
+    r = subprocess.run([sys.executable, "-c", GTSFM_BASES_SCRIPT, str(ref_modules.REF)], capture_output=True, text=True,
+                       check=True)
+    (OUT / "gtsfm_bases.json").write_text(r.stdout)
+
+
 def main():
     assert ref_modules.available(), "/root/reference is required"
     OUT.mkdir(parents=True, exist_ok=True)
@@ -433,6 +488,7 @@ def main():
     golden_lund_door()
     golden_retriever()
     golden_netvlad()
+    golden_gtsfm_bases()
 
 
 if __name__ == "__main__":
